@@ -14,6 +14,8 @@ host->device and device->host copies inside the timed region.
 N > 1 (torchrun): the SAME read set is sharded by read id across the ranks (strong scaling): bucket all-to-all over
 NCCL per LowHash iteration, all-gather of the k-mer ids, alignment of each rank's candidates.
 One JSON line is printed by rank 0.
+--dump-outputs DIR writes what the last timed step returned (see dump_outputs) as .npy files, so that two builds can be
+compared output for output on the same seeded input.
 """
 import argparse
 import json
@@ -260,6 +262,52 @@ def alignment_roofline(dp_cells, dp_ms, sm_mhz):
                            % (SM_COUNT, ALU_LANES_PER_SM, sm_mhz or 1965.0, ALU_OPS_PER_CELL)}
 
 
+# Caps of what --dump-outputs writes, for all ranks together: 54.1 MB at most (64 MB is the bound).
+DUMP_CANDIDATE_ROWS = 800_000         # 19.2 MB as float64
+DUMP_STATS_ROWS = 500_000             # 12 MB as float64
+DUMP_ALIGNMENT_ROWS = 80_000          # 10.24 MB as float64, and 0.64 MB of sizes
+DUMP_COMPRESSED_BYTES = 3_000_000     # 12 MB as float32
+
+
+def _sample_rows(n, cap, seed):
+    """All row indices when n <= cap, else a fixed seeded sample of cap of them, in order."""
+    if n <= cap:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, cap, replace=False))
+
+
+def dump_outputs(path, cand, stats=None, rec=None, ctoc=None, cdata=None, world=1):
+    """Writes the outputs of one step as float64 (exact for their 32-bit fields and counts) and float32 (bytes) arrays:
+      candidates.npy                 the LowHash0 candidates (readId0, readId1, isSameStrand), rows [n, 3]
+      read_lowhash_statistics.npy    the per-read LowHash0 statistics (ReadLowHashStatistics), rows [R, 3]
+      alignment_data.npy             the stored AlignmentData records, rows [n, 16]
+      compressed_alignment_sizes.npy the compressed-alignment byte count of each of those records
+      compressed_alignment_bytes.npy the compressed bytes of the first of those records, concatenated
+      counts.npy                     total candidates and alignments
+    Larger outputs are sampled: the same rows for the same counts. With `world` ranks each rank writes its own block of
+    the candidates and alignments within 1/world of their caps; the statistics, the same on every rank, are passed by
+    one rank only. All files together stay within the DUMP_* caps, 54.1 MB."""
+    os.makedirs(path, exist_ok=True)
+    ci = _sample_rows(len(cand), DUMP_CANDIDATE_ROWS // world, 1)
+    np.save(os.path.join(path, "candidates.npy"), np.asarray(cand)[ci].astype(np.float64))
+    counts = [len(cand)]
+    if stats is not None:
+        si = _sample_rows(len(stats), DUMP_STATS_ROWS, 3)
+        np.save(os.path.join(path, "read_lowhash_statistics.npy"), np.asarray(stats)[si].astype(np.float64))
+    if rec is not None:
+        ai = _sample_rows(len(rec), DUMP_ALIGNMENT_ROWS // world, 2)
+        ctoc = np.asarray(ctoc, np.int64)
+        sizes = ctoc[1:][ai] - ctoc[:-1][ai]
+        keep = int(np.searchsorted(np.cumsum(sizes), DUMP_COMPRESSED_BYTES // world, side="right"))
+        data = [cdata[ctoc[i]:ctoc[i + 1]] for i in ai[:keep]]
+        np.save(os.path.join(path, "alignment_data.npy"), np.asarray(rec)[ai].astype(np.float64))
+        np.save(os.path.join(path, "compressed_alignment_sizes.npy"), sizes.astype(np.float64))
+        np.save(os.path.join(path, "compressed_alignment_bytes.npy"),
+                np.concatenate(data).astype(np.float32) if data else np.zeros(0, np.float32))
+        counts.append(len(rec))
+    np.save(os.path.join(path, "counts.npy"), np.array(counts, np.float64))
+
+
 def effective_cpus():
     """Host CPUs this process can actually use: the affinity mask, capped by the container's CFS quota (cgroup v2 cpu.max or
     v1 cpu.cfs_quota_us / cpu.cfs_period_us). The pool's 1-GPU boxes show 128 logical CPUs under a quota of 16."""
@@ -318,6 +366,8 @@ def main():
     ap.add_argument("--no-align", action="store_true", help="LowHash0 only (profiling aid)")
     ap.add_argument("--align-method", type=int, default=3, choices=[3, 4],
                     help="3 = what Nanopore-May2022.conf selects (default); 4 = Align4, --Align.alignMethod 4")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (DIR/rank<r>/ with several GPUs)")
     args = ap.parse_args()
     wl = dict(WORKLOADS[args.workload])
     wl["align"] = dict(wl["align"], alignMethod=args.align_method)
@@ -422,18 +472,19 @@ def main():
                  "dp_ms": 0.0, "dp_cells": 0, "dp_useful_cells": 0, "alignments": 0}
     last = {}
 
-    def step(record, host_data7=None):
+    def step(record, host_data7=None, keep_outputs=False):
         """One pass of the hot path. host_data7 != None: end-to-end mode, the marker records come from (pinned) host
-        memory through shb_set_markers inside the timed region."""
+        memory through shb_set_markers inside the timed region. keep_outputs: leave the step's outputs in last["outputs"]
+        (only for the last step: held across steps they would keep the library from recycling its host result buffers)."""
         torch.cuda.synchronize()
         t0 = time.perf_counter()
         if host_data7 is not None:
             ctx.set_markers(dm.toc, host_data7, dm.flags, read_begin=rb, read_end=re, read_count_total=R, total_marker_count=M)
         if world == 1:
-            cand, _, _, res = ctx.lowhash0(lparams, want_stats=True)
+            cand, stats, _, res = ctx.lowhash0(lparams, want_stats=True)
             sweep_ms, sweep_launches, launches = res.sweepMs, res.sweepLaunches, res.kernelLaunches
         else:
-            cand, _, res = ctx.lowhash0_sharded(lparams, want_stats=True)
+            cand, stats, res = ctx.lowhash0_sharded(lparams, want_stats=True)
             if record:
                 tm = ctx.dist_timing()
                 for k in ("sweep", "partition", "exchange", "process", "final"):
@@ -446,6 +497,7 @@ def main():
         nal = 0
         d2h = len(cand) * 12
         t2 = t1
+        outputs = dict(cand=cand, stats=stats)
         if not args.no_align:
             t2 = time.perf_counter()
             if world > 1:           # gathers the k-mer ids of all ranks on the first call after the markers changed
@@ -455,6 +507,7 @@ def main():
             else:
                 rec, ctoc, cdata, ares = capi.compute_alignments(ctx, cand, aopts)
             nal = len(rec)
+            outputs.update(rec=rec, ctoc=ctoc, cdata=cdata)
             d2h += rec.nbytes + ctoc.nbytes + cdata.nbytes
             launches += ares.kernelLaunches
             last.update(alignment_data_digest=ares.alignmentDataDigest, compressed_digest=ares.compressedDigest,
@@ -475,6 +528,8 @@ def main():
             stats_acc["gather_s"] += t2 - t1
             stats_acc["align_s"] += t3 - t2
             stats_acc["alignments"] = nal
+        if keep_outputs:
+            last["outputs"] = outputs
         stats_acc["last_d2h"] = d2h
         return cand, nal
 
@@ -486,12 +541,18 @@ def main():
     with ClockSampler(local_rank) as clocks:
         ev0.record()
         t0 = time.perf_counter()
-        for _ in range(args.steps):
-            cand, nal = step(True)
+        for i in range(args.steps):
+            cand, nal = step(True, keep_outputs=bool(args.dump_outputs) and i == args.steps - 1)
         ev1.record()
         barrier()
         wall = time.perf_counter() - t0
     wall = allmax(wall)
+    if args.dump_outputs:
+        outputs = last.pop("outputs")
+        if rank != 0:
+            outputs["stats"] = None         # all-reduced: every rank holds the same statistics
+        dump_outputs(args.dump_outputs if world == 1 else os.path.join(args.dump_outputs, f"rank{rank}"), world=world, **outputs)
+        del outputs
     total_cand = allsum(len(cand))
     total_al = allsum(nal)
     # Per-rank view of the timed steps (the aggregate keys below are maxima over the ranks, which do not add up): host-clock
@@ -519,7 +580,7 @@ def main():
         host = torch.empty(M_local * 7, dtype=torch.uint8, pin_memory=True)
         data7 = host.numpy()
         dm.data7_to_host(out=data7)
-        e2e_steps = max(2, args.steps)
+        e2e_steps = args.steps
         step(False, host_data7=data7)
         barrier()
         t0 = time.perf_counter()

@@ -1,12 +1,13 @@
 """The `shasta.Assembler`-shaped facade (shasta_b200/assembler.py) and the reference's Data/ file formats.
 
-CPU part: files written by the facade's writer are opened by the reference's own MemoryMapped::Vector code
-(oracle/_ref) with the right record types, and files written by the reference (Markers, ReadFlags, Kmers from
-TinyTest through ReadLoader + MarkerFinder) are read back by the facade's reader.
-GPU part: the two entry points run on a reference-written Data/ directory with the reference's Python-script call
-sequence (scripts/FindAlignmentCandidatesLowHash0.py, scripts/ComputeAlignments.py) and reproduce the TinyTest pin."""
-import gzip
+CPU part: files written by the facade's writer are byte for byte the files the reference's own MemoryMapped::Vector code
+accepted with the right record types, and files written by the reference (Markers, ReadFlags, Kmers from TinyTest through
+ReadLoader + MarkerFinder) are read back by the facade's reader. What the reference did is stored in tests/golden/ref_golden.npz
+(tests/golden/make_ref_golden.py).
+GPU part: the two entry points run on a Data/ directory with the reference's Python-script call sequence
+(scripts/FindAlignmentCandidatesLowHash0.py, scripts/ComputeAlignments.py) and reproduce the TinyTest pin."""
 import os
+import sys
 
 import numpy as np
 import pytest
@@ -14,44 +15,45 @@ import pytest
 from oracle import bindings as B
 from shasta_b200 import assembler as A
 
-
-def fnv(raw):
-    h = 1469598103934665603
-    for b in bytes(raw):
-        h = ((h ^ b) * 1099511628211) & 0xFFFFFFFFFFFFFFFF
-    return h
+sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
+import make_ref_golden as RG  # noqa: E402
 
 
-@pytest.mark.skipif(not B.have_ref(), reason="reference build absent")
-def test_writer_is_readable_by_the_reference(tmp_path):
-    rng = np.random.default_rng(1)
-    cases = [(12, rng.integers(0, 1000, (1000, 3)).astype(np.uint32)), (64, rng.integers(0, 2**31, (77, 16)).astype(np.uint32)),
-             (24, rng.integers(0, 2**40, (50, 3)).astype(np.uint64)), (1, rng.integers(0, 255, 5000).astype(np.uint8)),
-             (8, rng.integers(0, 2**50, 4097).astype(np.uint64)), (4, np.zeros(0, np.uint32))]
-    for i, (size, arr) in enumerate(cases):
+def test_writer_is_readable_by_the_reference(tmp_path, golden_dir):
+    g = np.load(os.path.join(golden_dir, "ref_golden.npz"))
+    for i, (size, arr) in enumerate(RG.writer_cases()):
         path = str(tmp_path / f"v{i}")
         A.mm_write_vector(path, arr, object_size=size)
-        n, h = B.ref_open_vector(path, size)
-        assert n == arr.nbytes // size
-        assert h == fnv(arr.tobytes())
+        # the reference opened exactly these bytes as a Vector of `size`-byte records, with this count and payload checksum
+        assert np.array_equal(RG.sha256(open(path, "rb").read()), g["writer_sha256"][i])
+        assert g["writer_count"][i] == arr.nbytes // size
+        assert g["writer_checksum"][i] == RG.fnv(arr.tobytes())
         back = A.mm_read_vector(path, arr.dtype, object_size=size)
         assert np.array_equal(np.asarray(back).reshape(arr.shape), arr)
-    # wrong record size is rejected by the reference ("unexpected object size")
-    with pytest.raises(RuntimeError):
-        B.ref_open_vector(str(tmp_path / "v0"), 64)
+    # a wrong record size is rejected, as the reference's accessExistingReadOnly rejected v0 opened as 64-byte records
+    with pytest.raises(RuntimeError, match="object size"):
+        A.mm_read_vector(str(tmp_path / "v0"), np.uint8, object_size=64)
 
 
 @pytest.fixture(scope="module")
 def tiny_data_dir(tmp_path_factory):
-    if not B.have_ref() or not os.path.exists("/root/reference/tests/TinyTest.fasta.gz"):
-        pytest.skip("needs the reference tree")
-    d = tmp_path_factory.mktemp("run")
-    fasta = str(d / "TinyTest.fasta")
-    with open(fasta, "wb") as f:
-        f.write(gzip.open("/root/reference/tests/TinyTest.fasta.gz").read())
-    os.makedirs(d / "Data")
-    B.ref_write_data_dir(fasta, str(d / "Data") + "/", k=10)
-    return str(d / "Data") + "/"
+    """The Data/ files the reference writes for TinyTest, rebuilt from their stored headers and the golden markers. The payload
+    of Kmers is not stored: the reader needs only its header and size."""
+    g = np.load(os.path.join(os.path.dirname(__file__), "golden", "ref_golden.npz"))
+    z = np.load(os.path.join(os.path.dirname(__file__), "golden", "tinytest_markers.npz"))
+    d = tmp_path_factory.mktemp("run") / "Data"
+    os.makedirs(d)
+    payloads = {"Markers.toc": z["toc"], "Markers.data": z["data"], "ReadFlags": z["flags"], "Kmers": np.zeros(0, np.uint8)}
+    for name, payload in payloads.items():
+        key = name.replace(".", "_")
+        header = g[f"datadir_{key}_header"]
+        raw = header.tobytes() + bytes(4096 - header.nbytes) + payload.tobytes()
+        raw += bytes(int(header[5]) - len(raw))         # header word 5: fileSize
+        if name != "Kmers":
+            assert np.array_equal(RG.sha256(raw), g[f"datadir_{key}_sha256"]), name
+        with open(d / name, "wb") as f:
+            f.write(raw)
+    return str(d) + "/"
 
 
 def test_reader_on_reference_written_files(tiny_data_dir, golden_dir):

@@ -35,3 +35,26 @@ def test_effective_cpus_and_placement_helpers():
             def get_device_properties(i):
                 raise RuntimeError("no device")
     assert bench.gpu_numa_cpus(NoCuda, 0) == (None, None)
+
+
+def test_dump_outputs_stays_within_64_mb_at_every_world_size(tmp_path):
+    import numpy as np
+    rng = np.random.default_rng(0)
+    cand = rng.integers(0, 2**31, (3_000_000, 3)).astype(np.uint32)
+    stats = rng.integers(0, 2**40, (1_000_000, 3)).astype(np.uint64)
+    rec = rng.integers(0, 2**32, (300_000, 16), dtype=np.uint64).astype(np.uint32)
+    ctoc = np.concatenate([[0], np.cumsum(rng.integers(20, 400, len(rec)))]).astype(np.uint64)
+    cdata = rng.integers(0, 256, int(ctoc[-1])).astype(np.uint8)
+    for world in (1, 2, 8):
+        root = tmp_path / f"w{world}"
+        for rank in range(world):       # as bench.py calls it: the statistics come from one rank
+            bench.dump_outputs(str(root / f"rank{rank}"), cand, stats if rank == 0 else None, rec, ctoc, cdata, world=world)
+        total = sum(f.stat().st_size for f in root.rglob("*.npy"))
+        assert total <= 64_000_000, (world, total)
+    z = np.load(tmp_path / "w1" / "rank0" / "read_lowhash_statistics.npy")
+    assert z.dtype == np.float64 and z.shape == (bench.DUMP_STATS_ROWS, 3)
+    assert np.array_equal(z, stats[bench._sample_rows(len(stats), bench.DUMP_STATS_ROWS, 3)].astype(np.float64))
+    again = tmp_path / "again"
+    bench.dump_outputs(str(again), cand, stats, rec, ctoc, cdata)
+    for f in (tmp_path / "w1" / "rank0").iterdir():
+        assert np.array_equal(np.load(f), np.load(again / f.name)), f.name

@@ -1,10 +1,11 @@
 """GPU parity test of the device MarkerFinder (csrc/markers.cu, shb_find_markers) through the C ABI:
   * TinyTest: inputs and expected output both produced by the UNMODIFIED reference (tests/golden/tinytest_reads.npz ->
     tests/golden/tinytest_markers.npz, 124 036 markers), 7-byte records and toc bit for bit;
-  * a synthetic FASTA run through the reference's own ReadLoader + MarkerFinder live (oracle/_ref travels to the GPU box);
+  * synthetic FASTA files run through the reference's own ReadLoader + MarkerFinder (tests/golden/ref_golden.npz);
   * edge cases: reads shorter than k, empty reads, one read, k-mers straddling 64-base blocks at every offset;
   * the markers left on the device feed LowHash0 directly (no shb_set_markers): same candidates as from the uploaded records."""
 import os
+import sys
 
 import numpy as np
 import pytest
@@ -13,6 +14,8 @@ from oracle import bindings as B
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+import make_ref_golden as RG  # noqa: E402
 
 
 @pytest.fixture(scope="module")
@@ -49,18 +52,15 @@ def test_tinytest_markers_bit_for_bit(ctx):
     assert len(cand) == 186 and B.candidate_digest(cand) == 0x3fc2c96e354f8733
 
 
-@pytest.mark.skipif(not B.have_ref(), reason="reference build absent")
 @pytest.mark.parametrize("k", [6, 10, 14])
-def test_synthetic_fasta_against_live_reference(ctx, tmp_path, k):
-    from test_oracle_markers import write_synthetic_fasta
-    fasta = str(tmp_path / "synthetic.fasta")
-    write_synthetic_fasta(fasta, reads=60, seed=k)
-    r = B.ref_reads_from_fasta(fasta, k=k, min_read_length=1000)
-    m = B.ref_markers_from_fasta(fasta, k=k, min_read_length=1000)
+def test_synthetic_fasta_against_live_reference(ctx, k):
+    g = np.load(os.path.join(ROOT, "tests", "golden", "ref_golden.npz"))
+    name = f"fasta60_s{k}_k{k}"
+    r = RG.fasta_case(g, name)
     bitmap = np.packbits(r["is_marker"], bitorder="little").view(np.uint32)
-    toc, data, res = ctx.find_markers(k, r["word_offsets"], r["words"], r["base_counts"], m["flags"], is_marker_bitmap=bitmap)
-    assert res.markerCount == int(m["toc"][-1]) > 1000
-    assert np.array_equal(toc, m["toc"]) and np.array_equal(data, m["data"])
+    toc, data, res = ctx.find_markers(k, r["word_offsets"], r["words"], r["base_counts"], r["flags"], is_marker_bitmap=bitmap)
+    assert res.markerCount == int(g[f"fasta_{name}_toc"][-1]) > 1000
+    RG.assert_markers_match(g, name, toc, data)
 
 
 def _pack_reads(reads):

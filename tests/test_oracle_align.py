@@ -1,5 +1,5 @@
-"""CPU tests: the alignment oracle (oracle/align_oracle.c) against the reference's golden vectors and, where the
-reference build is available (oracle/_ref: unmodified Align4.cpp / Alignment.cpp / compressAlignment.cpp), against it.
+"""CPU tests: the alignment oracle (oracle/align_oracle.c) against the reference's golden vectors, among them outputs of the
+unmodified Align4.cpp / Alignment.cpp / compressAlignment.cpp stored in tests/golden.
 
 The overlap DP's tie-break rule is 'parity unpinned' (SeqAn absent, SURVEY.md F4); what IS pinned here:
   * shasta::compress bytes of the reference's own test vectors (SURVEY.md Appendix D),
@@ -7,11 +7,16 @@ The overlap DP's tie-break rule is 'parity unpinned' (SeqAn absent, SURVEY.md F4
   * the whole Align4 front end (cells, searches, components, band, selection) against the compiled Align4.cpp,
   * DP optimality properties that hold for any correct implementation (score = brute force, path validity).
 """
+import os
+import sys
+
 import numpy as np
-import pytest
 
 from oracle import bindings as B
 from shasta_b200 import synth
+
+sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
+import make_ref_golden as RG  # noqa: E402
 
 # src/compressAlignment.cpp:161-192 (testAlignmentCompression): 30 ordinal pairs exercising Formats 0-4.
 COMPRESSION_TEST_VECTOR = [
@@ -26,27 +31,17 @@ def test_compress_worked_example():
     assert np.array_equal(B.oracle_decompress(B.oracle_compress(o)), o)
 
 
-@pytest.mark.skipif(not B.have_ref(), reason="reference build absent")
-def test_reference_selftest_and_compress_vectors():
-    assert B._rlib().ref_test_alignment_compression() == 0
-    rng = np.random.default_rng(1)
-    for trial in range(200):
-        n = int(rng.integers(1, 60))
-        # streaks with skips spanning all five formats
-        scale = [3, 7, 500, 500000, 3000000][trial % 5]
-        x = np.cumsum(rng.integers(1, scale + 1, n)).astype(np.uint32)
-        y = np.cumsum(rng.integers(1, scale + 1, n)).astype(np.uint32)
-        run = rng.integers(0, 2, n).astype(bool)
-        for i in range(1, n):
-            if run[i]:
-                x[i:] -= x[i] - x[i - 1] - 1
-                y[i:] -= y[i] - y[i - 1] - 1
-        o = np.stack([x, y], 1)
-        assert np.array_equal(B.oracle_compress(o), B.ref_compress(o))
+def test_reference_selftest_and_compress_vectors(golden_dir):
+    # shasta::compress bytes of the reference for the ordinals of its own testAlignmentCompression and for seeded runs
+    # (tests/golden/make_ref_golden.py)
+    g = np.load(os.path.join(golden_dir, "ref_golden.npz"))
+    o = g["selftest_ordinals"]
+    assert np.array_equal(B.oracle_compress(o), g["selftest_compressed"])
+    assert np.array_equal(B.oracle_decompress(g["selftest_compressed"]), o)
+    toc = g["compress_toc"]
+    for i, o in enumerate(RG.compress_cases()):
+        assert np.array_equal(B.oracle_compress(o), g["compress_bytes"][int(toc[i]):int(toc[i + 1])])
         assert np.array_equal(B.oracle_decompress(B.oracle_compress(o)), o)
-    # Format 4 (|skip| >= 2^19) and a negative skip
-    o = np.array([[2000000, 5], [2000001, 6], [2000010, 1000000]], np.uint32)
-    assert np.array_equal(B.oracle_compress(o), B.ref_compress(o))
 
 
 def _brute_score(a, b, match, mismatch, gap, band=None):
@@ -97,26 +92,26 @@ def _pairs(d, cand, limit):
         yield km[toc[o0]:toc[o0 + 1]], km[toc[o1]:toc[o1 + 1]]
 
 
-@pytest.mark.skipif(not B.have_ref(), reason="reference build absent")
-def test_align4_front_end_matches_compiled_reference():
-    d = synth.generate(synth.SynthParams(reads=150, k=10, genome_markers=9000, n50_bases=9000, min_bases=5000, seed=5))
-    lp = B.LowHashParams(m=4, hashFraction=0.02, minHashIterationCount=6, minBucketSize=2, maxBucketSize=30, minFrequency=2)
-    cand, _, _ = B.oracle_lowhash0(d["toc"], d["data"], d["flags"], lp)
-    assert len(cand) > 100
-    for opts in (dict(maxSkip=100, maxDrift=100, maxTrim=100, minAlignedMarkerCount=10, minAlignedFraction=0.1),
-                 dict(maxSkip=30, maxDrift=30, maxTrim=30, minAlignedMarkerCount=60, minAlignedFraction=0.4,
-                      align4DeltaX=100, align4DeltaY=5, align4MinEntryCountPerCell=4, align4MaxDistanceFromBoundary=50, maxBand=300)):
+def test_align4_front_end_matches_compiled_reference(golden_dir):
+    # Align4 ordinals, AlignmentInfo words and compress bytes of the compiled reference on the same pairs
+    # (tests/golden/make_ref_golden.py)
+    g = np.load(os.path.join(golden_dir, "ref_golden.npz"))
+    pairs = RG.align4_pairs()
+    for j, opts in enumerate(RG.ALIGN4_OPTIONS):
         o4 = B.make_align_options(alignMethod=4, k=10, **opts)
+        ctoc = g[f"align4_{j}_comp_toc"]
         nonempty = 0
-        for a, b in _pairs(d, cand, 60):
+        for p, (a, b) in enumerate(pairs):
             st, al, tie = B.oracle_align_pair(a, b, o4)
-            ra = B.ref_align4(a, b, o4)
+            rbytes = g[f"align4_{j}_comp"][int(ctoc[p]):int(ctoc[p + 1])]
+            ra = B.oracle_decompress(rbytes)        # the reference's ordinals, stored in its compressed form
             if not tie:     # ties between kept components: the reference's pick depends on unordered_map order
                 assert np.array_equal(al, ra)
             if len(al):
                 nonempty += 1
-                assert np.array_equal(B.oracle_alignment_info(al, len(a), len(b)), B.ref_alignment_info(al, len(a), len(b)))
-                assert np.array_equal(B.oracle_compress(al), B.ref_compress(al))
+            if len(ra):
+                assert np.array_equal(B.oracle_alignment_info(ra, len(a), len(b)), g[f"align4_{j}_info"][p])
+                assert np.array_equal(B.oracle_compress(ra), rbytes)
         assert nonempty > 10
 
 

@@ -3,7 +3,8 @@
 Golden material (SURVEY.md section 8c / Appendix B, D):
   * MurmurHash64A / MurmurHash2 known answers computed from the reference's src/MurmurHash2.cpp;
   * the feature enumeration example of docs/ComputationalMethods.html:750-765;
-  * LowHash0 outputs of the unmodified reference on TinyTest and synthetic inputs (tests/golden).
+  * LowHash0 outputs of the unmodified reference on TinyTest and synthetic inputs (tests/golden), with parameters of the
+    configurations and away from them.
 """
 import json
 import os
@@ -17,6 +18,7 @@ from shasta_b200 import synth
 
 sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
 import make_golden as MG  # noqa: E402
+import make_ref_golden as RG  # noqa: E402
 
 
 def test_murmurhash64a_known_answers():
@@ -97,13 +99,11 @@ def test_bucket_count_too_small_raises(golden_dir):
         B.oracle_lowhash0(z["toc"], z["data"], z["flags"], B.LowHashParams(log2MinHashBucketCount=5))
 
 
-@pytest.mark.skipif(not B.have_ref(), reason="reference build absent")
-def test_oracle_matches_live_reference_random_params():
-    # Fresh (non-golden) comparison against the live reference build, when it is available.
-    d = synth.generate(synth.SynthParams(reads=150, k=10, genome_markers=20000, n50_bases=12000, min_bases=6000, seed=99))
-    for params in (dict(m=2, hashFraction=0.03, minHashIterationCount=3, minBucketSize=0, maxBucketSize=5, minFrequency=1),
-                   dict(m=7, hashFraction=0.1, minHashIterationCount=2, minBucketSize=3, maxBucketSize=40, minFrequency=2)):
-        p = B.LowHashParams(**params)
-        rc, rs, rit, _ = B.ref_lowhash0(d["toc"], d["data"], d["flags"], p, threads=3)
-        oc, os_, oit = B.oracle_lowhash0(d["toc"], d["data"], d["flags"], p)
-        assert np.array_equal(rc, oc) and np.array_equal(rs, os_) and np.array_equal(rit, oit)
+def test_oracle_matches_live_reference_random_params(golden_dir):
+    # Parameters away from the configurations, against the reference build's outputs (tests/golden/make_ref_golden.py).
+    g = np.load(os.path.join(golden_dir, "ref_golden.npz"))
+    d = RG.lowhash_random_input()
+    for j, params in enumerate(RG.LOWHASH_RANDOM_PARAMS):
+        oc, os_, oit = B.oracle_lowhash0(d["toc"], d["data"], d["flags"], B.LowHashParams(**params))
+        assert np.array_equal(g[f"lowhash_{j}_candidates"], oc) and np.array_equal(g[f"lowhash_{j}_stats"], os_)
+        assert np.array_equal(g[f"lowhash_{j}_summary"], oit)

@@ -1,14 +1,16 @@
 """CPU test: the marker-finding oracle (oracle/markers_oracle.c) against the golden output of the UNMODIFIED reference
-MarkerFinder on TinyTest (tests/golden/tinytest_markers.npz; inputs tests/golden/tinytest_reads.npz), and — where the
-reference build is present — against the reference run live on a synthetic FASTA."""
+MarkerFinder on TinyTest (tests/golden/tinytest_markers.npz; inputs tests/golden/tinytest_reads.npz), and against the
+reference's ReadLoader + MarkerFinder on synthetic FASTA files (tests/golden/ref_golden.npz)."""
 import os
+import sys
 
 import numpy as np
-import pytest
 
 from oracle import bindings as B
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+import make_ref_golden as RG  # noqa: E402
 
 
 def _golden():
@@ -26,23 +28,10 @@ def test_marker_oracle_reproduces_reference_tinytest():
     assert np.array_equal(toc, m["toc"]) and np.array_equal(data, m["data"])
 
 
-def write_synthetic_fasta(path, reads=40, seed=3):
-    rng = np.random.default_rng(seed)
-    with open(path, "w") as f:
-        for i in range(reads):
-            n = int(rng.integers(10000, 14000))
-            # homopolymer runs of random length so that the run-length encoding has something to do
-            bases = np.repeat(rng.integers(0, 4, n), rng.integers(1, 4, n))[:n]
-            f.write(f">read{i}\n" + "".join("ACGT"[b] for b in bases) + "\n")
-
-
-@pytest.mark.skipif(not B.have_ref(), reason="reference build absent")
-def test_marker_oracle_against_live_reference(tmp_path):
-    fasta = str(tmp_path / "synthetic.fasta")
-    write_synthetic_fasta(fasta)
-    for k in (8, 10):
-        r = B.ref_reads_from_fasta(fasta, k=k, min_read_length=1000)
-        m = B.ref_markers_from_fasta(fasta, k=k, min_read_length=1000)
-        toc, data = B.oracle_find_markers(r["word_offsets"], r["words"], r["base_counts"], r["is_marker"], k)
+def test_marker_oracle_against_live_reference():
+    g = np.load(os.path.join(ROOT, "tests", "golden", "ref_golden.npz"))
+    for name in ("fasta40_s3_k8", "fasta40_s3_k10"):
+        r = RG.fasta_case(g, name)
+        toc, data = B.oracle_find_markers(r["word_offsets"], r["words"], r["base_counts"], r["is_marker"], r["k"])
         assert toc[-1] > 1000
-        assert np.array_equal(toc, m["toc"]) and np.array_equal(data, m["data"])
+        RG.assert_markers_match(g, name, toc, data)

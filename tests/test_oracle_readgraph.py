@@ -1,22 +1,16 @@
 """createReadGraph (ReadGraph.creationMethod 0) oracle against a direct statement of src/AssemblerReadGraph.cpp:35-175:
 per read, the maxAlignmentCount largest (markerCount, alignmentId) pairs; edges and connectivity in the reference's order."""
+import os
+import sys
+
 import numpy as np
 
 from oracle import bindings as B
 
+sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
+import make_ref_golden as RG  # noqa: E402
 
-def _records(rng, n, reads):
-    rec = np.zeros((n, 16), np.uint32)
-    a = rng.integers(0, reads, n)
-    b = rng.integers(0, reads, n)
-    same = a == b
-    b[same] = (a[same] + 1) % reads
-    rec[:, 0] = np.minimum(a, b)
-    rec[:, 1] = np.maximum(a, b)
-    rec[:, 2] = rng.integers(0, 2, n)
-    rec[:, 9] = rng.integers(10, 14, n)         # few distinct marker counts: ties are decided by the alignment id
-    rec[:, 15] = rng.integers(0, 2, n)          # stale flags must be overwritten
-    return rec
+_records = RG.records
 
 
 def _direct(rec, reads, k):
@@ -56,48 +50,23 @@ def test_against_direct_statement():
         assert np.all(edges[:, 0] < edges[:, 1]) if len(edges) else True
 
 
-def _quality_records(rng, n, reads):
-    """AlignmentData with plausible AlignmentInfo words: Data{markerCount, firstOrdinal, lastOrdinal} x 2, markerCount, offsets,
-    maxSkip, maxDrift."""
-    rec = _records(rng, n, reads)
-    for side in (0, 1):
-        total = rng.integers(200, 5000, n)
-        first = rng.integers(0, 150, n)
-        last = total - 1 - rng.integers(0, 150, n)
-        rec[:, 3 + 3 * side] = total
-        rec[:, 4 + 3 * side] = first
-        rec[:, 5 + 3 * side] = np.maximum(last, first)
-    span = np.minimum(rec[:, 5] - rec[:, 4], rec[:, 8] - rec[:, 7]) + 1
-    rec[:, 9] = np.maximum(1, (span * rng.uniform(0.2, 1.0, n)).astype(np.uint32))       # markerCount: up to ~4800 (beyond 3000)
-    rec[:, 13] = rng.integers(0, 140, n)        # maxSkip: some beyond the histogram's 100
-    rec[:, 14] = rng.integers(0, 120, n)        # maxDrift
-    return rec
+_quality_records = RG.quality_records
 
 
-import pytest
-
-
-@pytest.mark.skipif(not B.have_ref(), reason="reference build absent")
-def test_histogram2_and_indicators_against_the_reference_classes():
-    rng = np.random.default_rng(5)
-    for (start, stop, bins) in [(0, 1, 100), (0, 3000, 300), (0, 100, 100)]:
-        for trial in range(20):
-            n = int(rng.integers(0, 400))
-            # in range, exactly on the upper edge, and well beyond it (the dynamic-bounds growth path)
-            x = rng.uniform(start, stop * rng.choice([0.5, 1.0, 1.7]), n)
-            if n and trial % 3 == 0:
-                x[rng.integers(0, n)] = stop
-            x = np.round(x, 2) if stop > 1 else x
-            for fraction in (0.015, 0.12, 0.5, 0.88, 0.985, 1.0):
-                want = B.ref_histogram2_threshold(x, start, stop, bins, fraction)
-                got = B.oracle_histogram2_threshold(x, start, stop, bins, fraction)
-                assert want == got or (np.isnan(want) and np.isnan(got)), (start, stop, bins, trial, fraction)
+def test_histogram2_and_indicators_against_the_reference_classes(golden_dir):
+    # Thresholds of the reference's Histogram2 and its AlignmentInfo accessors (tests/golden/make_ref_golden.py)
+    g = np.load(os.path.join(golden_dir, "ref_golden.npz"))
+    cases, rng = RG.hist2_cases()
+    for i, (start, stop, bins, x) in enumerate(cases):
+        for fraction, want in zip(RG.HIST2_FRACTIONS, g["hist2_thresholds"][i]):
+            got = B.oracle_histogram2_threshold(x, start, stop, bins, fraction)
+            assert want == got or (np.isnan(want) and np.isnan(got)), (start, stop, bins, i, fraction)
     rec = _quality_records(rng, 200, 30)
-    for r in rec:
+    for r, want in zip(rec, g["hist2_indicators"]):
         d0, d1 = r[3:6].astype(np.int64), r[6:9].astype(np.int64)
         frac = min(r[9] / (d0[2] + 1 - d0[1]), r[9] / (d1[2] + 1 - d1[1]))
         trim = max(min(d0[1], d1[1]), min(d0[0] - 1 - d0[2], d1[0] - 1 - d1[2]))
-        assert np.array_equal(B.ref_alignment_indicators(r), np.array([frac, r[9], r[14], r[13], trim], np.float64))
+        assert np.array_equal(want, np.array([frac, r[9], r[14], r[13], trim], np.float64))
 
 
 def test_creation_method_2_against_direct_statement():

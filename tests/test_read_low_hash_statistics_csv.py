@@ -1,26 +1,24 @@
 """ReadLowHashStatistics.csv written by the facade against the file the reference's own LowHash0 leaves in its working directory
 (src/LowHash0.cpp:220-243)."""
 import os
+import sys
 
 import numpy as np
-import pytest
 
-from oracle import bindings as B
 from shasta_b200 import assembler as A
-from shasta_b200 import synth
+
+sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
+import make_ref_golden as RG  # noqa: E402
 
 
-@pytest.mark.skipif(not B.have_ref(), reason="reference build absent")
-def test_csv_is_byte_identical_to_the_reference(tmp_path, monkeypatch):
+def test_csv_is_byte_identical_to_the_reference(tmp_path, monkeypatch, golden_dir):
+    # the reference's per-read statistics and the file it wrote from them (tests/golden/make_ref_golden.py)
     monkeypatch.chdir(tmp_path)
-    monkeypatch.setenv("SHB_REF_KEEP_CSV", str(tmp_path))
-    d = synth.generate(synth.SynthParams(reads=300, k=10, genome_markers=30000, n50_bases=12000, min_bases=6000, seed=17,
-                                         palindromic_every=23))
-    for m, min_bucket, max_bucket in ((4, 2, 30), (3, 5, 8)):
-        p = B.LowHashParams(m=m, hashFraction=0.02, minHashIterationCount=6, minBucketSize=min_bucket, maxBucketSize=max_bucket,
-                            minFrequency=2)
-        _, stats, _, _ = B.ref_lowhash0(d["toc"], d["data"], d["flags"], p, threads=2)
-        want = open("ReadLowHashStatistics.csv").read()
+    g = np.load(os.path.join(golden_dir, "ref_golden.npz"))
+    d = RG.csv_input()
+    for i, (m, _, _) in enumerate(RG.CSV_CASES):
+        stats = g[f"csv_{i}_stats"]
+        want = g[f"csv_{i}_text"].tobytes().decode()
         A.write_read_low_hash_statistics_csv("ours.csv", stats, d["toc"], d["flags"], m)
         got = open("ours.csv").read()
         assert got == want
